@@ -2,6 +2,7 @@
 """bench.py -- SageBlock fwd+bwd throughput (BASELINE.json metric) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload batch|c4|c1|infer|c2] [--impl ours|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one training pass of the hot path over one batch: CSR build from a fresh
@@ -26,6 +27,11 @@ e2e     = the same through the public module call with pinned HOST inputs: H2D o
 roofline= the dominant kernel (longest share of the step), algorithmic bytes / its own
           CUDA-event time / measured HBM peak; roofline_step = SURVEY 8d's per-layer
           fwd+bwd byte model for the whole step.
+--dump-outputs DIR writes what the last timed step returned to its caller as DIR/<name>.npy (float32; rank 0's
+          share at N > 1), so that two builds run with the same arguments can be compared output for output:
+          out = block output, dx = gradient of x, grad.<parameter> = every parameter gradient (no dx / grad.* for
+          infer).  Of out and dx only a fixed, seeded sample of DUMP_ROWS rows is written (all rows of a smaller
+          output), at most 32 MB in all at width 128.  c2 writes the loss and every parameter after the Adam step.
 """
 from __future__ import annotations
 
@@ -70,6 +76,24 @@ WORKLOADS = {
 }
 SLOPE = 0.1
 METRIC = "sageblock_fwd_bwd_edges_per_sec"     # --workload infer reports forward-only traversals under the same name, flagged in config.step
+DUMP_ROWS = 32768
+
+
+def dump_rows(n):
+    """Row indices of the --dump-outputs sample of an [n, F] output: all rows when n <= DUMP_ROWS, else the same
+    seeded DUMP_ROWS rows (ascending) for every build and run."""
+    if n <= DUMP_ROWS:
+        return torch.arange(n)
+    return torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+
+
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: each tensor as dirname/<name>.npy, float64 kept, every other dtype as float32."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        np.save(os.path.join(dirname, name + ".npy"), t.numpy() if t.dtype == torch.float64 else t.float().numpy())
 
 
 def env_rank():
@@ -632,8 +656,10 @@ def main_ours(args, wl):
     # (~0.5 s of the same kernels, untimed for the headline), then the W warm-up steps, then the K timed steps.
     peak_gbs, peak_src = measured_peaks()
     kern = None if args.skip_kernel_timing else time_kernels(blk, batches[0]["x"].detach(), batches[0]["ei"], N, E, hdims, peak_gbs, batches[0]["bv"], batches[0]["graphs"])
+    # every step's output is held until the next one returns (the timed loop keeps the last for --dump-outputs), so the
+    # warm-up holds it the same way: the timed steps then find both output blocks in the caching allocator
     for i in range(max(3, args.warmup)):
-        step(batches[i % 2])
+        y = step(batches[i % 2])
     barrier()
     launches0 = _lib.lib.sldm_launch_count()
     t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -642,7 +668,7 @@ def main_ours(args, wl):
     t0.record()
     h0 = time.perf_counter()
     for i in range(args.steps):
-        step(batches[i % 2])
+        y = step(batches[i % 2])
     host_enqueue_ms = (time.perf_counter() - h0) * 1e3 / args.steps   # host time to ENQUEUE a step (no sync inside)
     t1.record()
     barrier()
@@ -650,6 +676,14 @@ def main_ours(args, wl):
     launches = _lib.lib.sldm_launch_count() - launches0
     ms_total = t0.elapsed_time(t1)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:        # before the e2e steps below overwrite the gradients
+        rows = dump_rows(y.size(0)).to(dev)
+        arrays = {"out": y.index_select(0, rows)}
+        if not fwd_only:
+            arrays["dx"] = batches[(args.steps - 1) % 2]["x"].grad.index_select(0, rows)
+            arrays.update({"grad." + k: p.grad for k, p in blk.named_parameters()})
+        dump_outputs(args.dump_outputs, arrays)
+    del y
 
     # ---- end to end: pinned host inputs -> H2D -> step -> D2H of the step's metric, every step ----
     # Input pipeline as a training loop would run it: the H2D copy of step i+1 is issued on a copy stream while
@@ -824,7 +858,13 @@ def main():
     ap.add_argument("--no-c4", action="store_true", help="skip the c4 sub-record of the default line")
     ap.add_argument("--skip-kernel-timing", action="store_true",
                     help="skip the per-kernel-group timing (used for the ncu launch list: only whole steps are launched)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.workload == "c2":                  # SURVEY 8(d) C2: the full GruSage training step, its own metric (bench_c2.py)
         import bench_c2
         return bench_c2.main(args)

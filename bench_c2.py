@@ -191,13 +191,17 @@ def main_ours(args):
     sampler.mark_begin()
     t0.record()
     for i in range(args.steps):
-        step(batches[i % 2]["dev"])
+        loss = step(batches[i % 2]["dev"])
     t1.record()
     barrier()
     sampler.mark_end()
     launches = _lib.lib.sldm_launch_count() - launches0
     ms_total = t0.elapsed_time(t1)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:        # the step's loss and the parameters its Adam step left behind
+        from bench import dump_outputs
+        dump_outputs(args.dump_outputs, {"loss": torch.tensor([loss], dtype=torch.float64),
+                                         **{"param." + k: p for k, p in model.named_parameters()}})
 
     # ---- end to end: the batch is copied from pinned host memory every step (prefetched one step ahead on a copy stream) ----
     copy_stream, main_stream = torch.cuda.Stream(device=dev), torch.cuda.current_stream(dev)
