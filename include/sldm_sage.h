@@ -320,7 +320,7 @@ int sldm_edge_build_fill(const float* x, int64_t V, int32_t T, int32_t F, float 
                          const int32_t* offsets, int64_t E, int64_t* edge_index, float* edge_attr,
                          sldm_stream_t stream);
 
-/* ---- sequence head: fused single-layer GRU, last hidden state ---------------
+/* ---- sequence head: fused GRU layers, last hidden state ----------------------
  * Replaces `gru_out, hlast = self.gru(x); x = hlast[-1]` (src/models/grusage.py:160-161; nn.GRU(input_size = dynamic
  * features, hidden_size, num_layers = 1, batch_first = True) built at grusage.py:55-60, h0 = 0) and its autograd
  * backward.  x [N,T,I] fp32 contiguous; W_ih [3H,I], W_hh [3H,H] (16-byte aligned), b_ih, b_hh [3H]: torch's
@@ -338,19 +338,54 @@ int sldm_edge_build_fill(const float* x, int64_t V, int32_t T, int32_t F, float 
  *              db_ih[g*H + 32u + lane]; v = 27U + u -> db_hh[2H + 32u + lane] (db_hh[:2H] = db_ih[:2H]), U = H/32.
  *   wgrad    : dW_hh = dgh^T . h_prev over the T*N rows (h_prev read in place from `saved`), as
  *              sldm_gru_wgrad_tiles(N, T) partial [3H,H] tiles (one per persistent CTA) the caller adds up.
+ *
+ * Stacked layers (nn.GRU(num_layers = L), no inter-layer dropout): layer l >= 1 reads the output sequence h^{l-1}_t of
+ * the layer below, W_ih_l is [3H,H]; only the last step of the last layer is consumed.  All sequence buffers are
+ * time-major: h_seq [T,N,H], gi / dgi [T,N,3H], dh_seq [T,N,H].  Per layer l >= 1:
+ *   forward  : sldm_gru_project_forward(h_seq^{l-1} -> gi), then sldm_gru_layer_forward with gi (x = NULL).
+ *   backward : sldm_gru_layer_backward (x = NULL, dh_seq = the gradient of h^l_t from the layer above or NULL,
+ *              dh_last NULL below the top) -> dgh, dgi; dW_hh by sldm_gru_wgrad; dW_ih by
+ *              sldm_gru_wgrad_strided(dgi, h_seq^{l-1}, stride H); the layer below's dh_seq by
+ *              sldm_gru_project_backward(dgi -> dY).
+ *   Layer 0 is the single-layer path plus h_seq (forward) and dh_seq (backward).
+ *   stack_supported : layer 0 within sldm_gru_supported(T, I, H); the layers above have no T limit.
+ *   layer_forward   : exactly one of x [N,T,I] (layer 0: W_ih [3H,I], b_ih used) or gi [T,N,3H] (16-byte aligned,
+ *                     b_ih included; W_ih, b_ih, I ignored).  h_last [N,H] may be NULL; saved as above (NULL for
+ *                     inference); h_seq [T,N,H] receives h_t of every step (NULL: not written).
+ *   layer_backward  : x NULL selects the deep mode (I ignored; the dW_ih slots of the partials are zeros, the bias
+ *                     slots as above).  dh_last [N,H] may be NULL (zeros); dh_seq [T,N,H] may be NULL; dgi_n as
+ *                     above; dgi [T,N,3H] (may be NULL) receives the input-side pre-activation gradients [dr dz dn].
+ *   project_forward : gi[r] = b_ih + h_seq[r] . W_ih^T over rows = T*N ([H] -> [3H]); project_backward:
+ *                     dy[r] = dgi[r] . W_ih ([3H] -> [H]).  W_ih [3H,H]; inputs 16-byte aligned.  FP32 FMA chains in
+ *                     sequential k order.
+ *   wgrad_strided   : sldm_gru_wgrad with the second operand's row stride given (a multiple of 4, >= H): 5H reads
+ *                     h_prev in place from `saved` (= sldm_gru_wgrad), H reads an h_seq (dW_ih = dgi^T . h_seq).
  */
 int     sldm_gru_supported(int32_t T, int32_t I, int32_t H);
+int     sldm_gru_stack_supported(int32_t T, int32_t I, int32_t H);
 int64_t sldm_gru_partial_rows(int64_t N);
 int64_t sldm_gru_partial_width(int32_t H);
 int     sldm_gru_forward(const float* x, int64_t N, int32_t T, int32_t I, int32_t H,
                          const float* W_ih, const float* W_hh, const float* b_ih, const float* b_hh,
                          float* h_last, float* saved, sldm_stream_t stream);
+int     sldm_gru_layer_forward(const float* x, const float* gi, int64_t N, int32_t T, int32_t I, int32_t H,
+                               const float* W_ih, const float* W_hh, const float* b_ih, const float* b_hh,
+                               float* h_last, float* saved, float* h_seq, sldm_stream_t stream);
 int     sldm_gru_backward(const float* x, int64_t N, int32_t T, int32_t I, int32_t H, const float* W_hh,
                           const float* dh_last, const float* saved, float* dgh, float* dgi_n, float* partials,
                           int64_t partial_rows, sldm_stream_t stream);
+int     sldm_gru_layer_backward(const float* x, int64_t N, int32_t T, int32_t I, int32_t H, const float* W_hh,
+                                const float* dh_last, const float* dh_seq, const float* saved, float* dgh,
+                                float* dgi_n, float* dgi, float* partials, int64_t partial_rows, sldm_stream_t stream);
+int     sldm_gru_project_forward(const float* h_seq, int64_t rows, int32_t H, const float* W_ih, const float* b_ih,
+                                 float* gi, sldm_stream_t stream);
+int     sldm_gru_project_backward(const float* dgi, int64_t rows, int32_t H, const float* W_ih, float* dy,
+                                  sldm_stream_t stream);
 int64_t sldm_gru_wgrad_tiles(int64_t N, int32_t T);
 int     sldm_gru_wgrad(const float* dgh, const float* saved, int64_t N, int32_t T, int32_t H,
                        float* partials, int64_t partial_tiles, sldm_stream_t stream);
+int     sldm_gru_wgrad_strided(const float* dg, const float* a, int64_t a_stride, int64_t N, int32_t T, int32_t H,
+                               float* partials, int64_t partial_tiles, sldm_stream_t stream);
 
 /* ---- whole block, host buffers in / host buffers out -----------------------
  * For hosts that own no device memory (the reference-side stub in

@@ -83,6 +83,12 @@ _PROTOS = {
     "sldm_gru_backward": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _p, _p, _p, _p, _i64, _p]),
     "sldm_gru_wgrad_tiles": (_i64, [_i64, _i32]),
     "sldm_gru_wgrad": (C.c_int, [_p, _p, _i64, _i32, _i32, _p, _i64, _p]),
+    "sldm_gru_stack_supported": (C.c_int, [_i32, _i32, _i32]),
+    "sldm_gru_layer_forward": (C.c_int, [_p, _p, _i64, _i32, _i32, _i32, _p, _p, _p, _p, _p, _p, _p, _p]),
+    "sldm_gru_layer_backward": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p]),
+    "sldm_gru_project_forward": (C.c_int, [_p, _i64, _i32, _p, _p, _p, _p]),
+    "sldm_gru_project_backward": (C.c_int, [_p, _i64, _i32, _p, _p, _p]),
+    "sldm_gru_wgrad_strided": (C.c_int, [_p, _p, _i64, _i64, _i32, _i32, _p, _i64, _p]),
     "sldm_sage_block_forward_host": (C.c_int, [_p, _p, _i64, _i64, C.POINTER(_i32), _i32, C.POINTER(_p), _f, _f, _p]),
     "sldm_sage_block_train_host": (C.c_int, [_p, _p, _i64, _i64, C.POINTER(_i32), _i32, C.POINTER(_p), _f, _f,
                                              _p, _p, _p, C.POINTER(_p)]),

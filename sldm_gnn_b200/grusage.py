@@ -22,7 +22,7 @@ import os
 import torch
 import torch.nn as nn
 
-from .gru import fused_gru_eligible, gru_last_hidden
+from .gru import fused_gru_eligible, fused_gru_stack_eligible, gru_last_hidden, gru_stack_last_hidden
 from .map_attention import MapSpatialAttention
 from .ops import index_checks
 from .readout import global_max_pool, global_mean_max_pool, global_mean_pool
@@ -158,16 +158,21 @@ class GruSage(nn.Module):
 
         Default: the fused kernels of csrc/gru.cu (all T steps of a tile of sequences on one SM; gru.py) whenever the
         module is one batch-first layer with hidden 32 / 64 / 96 and at most 8 input features -- the reference's
-        configuration (main.py:42-44: hidden 96, one layer, 6 dynamic features).  Anything else, or
-        SLDM_DISABLE_FUSED_GRU=1, goes through torch's library GRU, and there through ATen's native path (one cuBLAS
+        configuration (main.py:42-44: hidden 96, one layer, 6 dynamic features).  A stacked head (gru_num_layers > 1)
+        with the same limits on its first layer runs on the same kernels layer by layer (gru_stack_last_hidden: the
+        layers above take their input projection from k_gru_proj and have no limit on T), unless inter-layer dropout
+        is active in training.  Anything else, or SLDM_DISABLE_FUSED_GRU=1, goes through torch's library GRU, and there through ATen's native path (one cuBLAS
         GEMM + one fused cell kernel per step) rather than cuDNN's: measured on B200 at the C2 shape (205 k sequences
         x 16 frames, input 6, hidden 96) the native path takes 35 ms forward + backward against 118 ms, and it computes
         in true fp32 -- cuDNN's RNN runs TF32 under torch's default flags (2e-4 off the CPU result,
         tools/gru_probe.py), which is outside this package's 1e-5 bar.  cuDNN also indexes its gate workspace
         (N * T * 3H elements) with 32 bits and faults beyond 2^31; sequences are independent, so very large batches go
         through the library path in slices -- same numbers, no limit."""
-        if os.environ.get("SLDM_DISABLE_FUSED_GRU", "0") != "1" and fused_gru_eligible(self.gru, x):
-            return gru_last_hidden(self.gru, x)
+        if os.environ.get("SLDM_DISABLE_FUSED_GRU", "0") != "1":
+            if fused_gru_eligible(self.gru, x):
+                return gru_last_hidden(self.gru, x)
+            if fused_gru_stack_eligible(self.gru, x):
+                return gru_stack_last_hidden(self.gru, x)
         n, per_seq = x.size(0), x.size(1) * 3 * self.gru.hidden_size
         rows = max(1, (1 << 30) // max(per_seq, 1))
         with torch.backends.cudnn.flags(enabled=False):
