@@ -326,7 +326,8 @@ int sldm_edge_build_fill(const float* x, int64_t V, int32_t T, int32_t F, float 
  * backward.  x [N,T,I] fp32 contiguous; W_ih [3H,I], W_hh [3H,H] (16-byte aligned), b_ih, b_hh [3H]: torch's
  * weight_ih_l0 / weight_hh_l0 / bias_ih_l0 / bias_hh_l0, gates ordered (r, z, n).  Same formulas as ATen's fused cell.
  *   supported: H in {32, 64, 96}, I <= 8, T*I small enough for the shared-memory tile (sldm_gru_supported() != 0);
- *              anything else returns SLDM_EUNSUPPORTED (the host module then keeps torch's library GRU).
+ *              anything else returns SLDM_EUNSUPPORTED (the host module then takes the projected path below, or
+ *              keeps torch's library GRU).
  *   forward  : h_last [N,H].  Training: saved [T,N,5,H] (NULL for inference) receives, per step and sequence,
  *              h_{t-1} | r | z | n | W_hn h + b_hn -- what backward needs (time-major so that a tile's stores of one
  *              step are contiguous).
@@ -360,6 +361,18 @@ int sldm_edge_build_fill(const float* x, int64_t V, int32_t T, int32_t F, float 
  *                     sequential k order.
  *   wgrad_strided   : sldm_gru_wgrad with the second operand's row stride given (a multiple of 4, >= H): 5H reads
  *                     h_prev in place from `saved` (= sldm_gru_wgrad), H reads an h_seq (dW_ih = dgi^T . h_seq).
+ *
+ * Projected layer 0 (sequences too long or inputs too wide for the x tile above): layer 0 is fed like the layers
+ * above it, through gi, so neither T nor the tile limits it.
+ *   projected_supported   : H in {32, 64, 96} and 1 <= I <= 128 (W_ih is held in shared memory); no limit on T.
+ *   input_project_forward : gi[t][n][:] = b_ih + W_ih . x[n][t][:], x [N,T,I] batch-first -> gi [T,N,3H] time-major;
+ *                           then sldm_gru_layer_forward with gi.  W_ih [3H,I].  FP32 FMA chains in sequential k
+ *                           order, starting from the bias.
+ *   backward              : sldm_gru_layer_backward in the deep mode (x = NULL) -> dgh, dgi and the bias partials;
+ *                           dW_hh by sldm_gru_wgrad; dW_ih by sldm_gru_input_wgrad.
+ *   input_wgrad           : dW_ih [3H,I] = sum over the T*N rows of dgi[t][n]^T . x[n][t], as the first
+ *                           sldm_gru_wgrad_tiles(N, T) partial [3H,I] tiles of `partials` (the caller adds them up; a
+ *                           fixed order, so the sum is the same run to run).  dgi 16-byte aligned.
  */
 int     sldm_gru_supported(int32_t T, int32_t I, int32_t H);
 int     sldm_gru_stack_supported(int32_t T, int32_t I, int32_t H);
@@ -386,6 +399,11 @@ int     sldm_gru_wgrad(const float* dgh, const float* saved, int64_t N, int32_t 
                        float* partials, int64_t partial_tiles, sldm_stream_t stream);
 int     sldm_gru_wgrad_strided(const float* dg, const float* a, int64_t a_stride, int64_t N, int32_t T, int32_t H,
                                float* partials, int64_t partial_tiles, sldm_stream_t stream);
+int     sldm_gru_projected_supported(int32_t I, int32_t H);
+int     sldm_gru_input_project_forward(const float* x, int64_t N, int32_t T, int32_t I, int32_t H,
+                                       const float* W_ih, const float* b_ih, float* gi, sldm_stream_t stream);
+int     sldm_gru_input_wgrad(const float* dgi, const float* x, int64_t N, int32_t T, int32_t I, int32_t H,
+                             float* partials, int64_t partial_tiles, sldm_stream_t stream);
 
 /* ---- whole block, host buffers in / host buffers out -----------------------
  * For hosts that own no device memory (the reference-side stub in

@@ -22,10 +22,14 @@
 // k_gru_fwd's gi mode; backward, k_gru_bwd's deep mode takes the per-step upstream gradient dh_seq and writes
 // dgi [T,N,3H], from which k_gru_wgrad gives dW_ih (against h_seq) and k_gru_proj the layer below's dh_seq.
 //
+// Projected layer 0 (sequences too long, or inputs too wide, for the x tile): k_gru_xproj projects x into gi and layer 0
+// runs the gi mode / deep mode like the layers above; k_gru_xwgrad gives its dW_ih = dgi^T x.
+//
 // Arithmetic: FP32 FMA in sequential k order, expf / tanhf / IEEE division like ATen's gru_cell_forward, i.e. the
 // reference's own formulas (aten/src/ATen/native/cuda/RNN.cu); bound by the FP32 pipe (2*3H*H flops per sequence and
-// step each way), not by HBM.  Limits: H in {32, 64, 96}, layer 0's input width <= 8 and its x tile must fit shared
-// memory; the layers above have no limit on T.
+// step each way), not by HBM.  Limits: H in {32, 64, 96}; on the tile path layer 0's input width <= 8 and its x tile
+// must fit shared memory; on the projected path layer 0's input width <= kGruMaxProjI = 128 and no limit on T; the
+// layers above have no limit on T.
 #include "common.cuh"
 #include <algorithm>
 
@@ -558,6 +562,173 @@ k_gru_proj(const float* __restrict__ in, int64_t rows, const float* __restrict__
   }
 }
 
+// Layer-0 input projection for sequences too long (or inputs too wide) for the x tile of k_gru_fwd / k_gru_bwd:
+//   gi[t][n][:] = b_ih + W_ih . x[n][t][:]   (batch-first x [N,T,I] -> time-major gi [T,N,3H], the layout of the gi mode).
+// One CTA per tile of 64 sequences walks the steps; W_ih sits in shared memory as Ws[n][k] (odd row stride I|1:
+// conflict-free scalar loads with lane = output column) and the tile's rows of x are streamed kGruXRow floats per row at
+// a time (a chunk of whole steps), so nothing depends on T.  A warp owns 8 rows (read as broadcasts), a lane 3H/32
+// output columns; the 64 x 3H outputs of a step are one contiguous range of gi.  Each output is one FP32 FMA chain in
+// sequential k order starting from the bias, as in k_gru_proj.  I <= kGruMaxProjI = 128: W_ih takes 288 x 129 floats
+// (149 KB) at H = 96, the x chunk 32 KB.
+constexpr int kGruMaxProjI = 128;
+constexpr int kGruXRow = 128;     // floats of x per sequence and chunk (at least one step)
+
+template <int H>
+__global__ void __launch_bounds__(kGruThreads, 2)
+k_gru_xproj(const float* __restrict__ x, int64_t N, int T, int I, const float* __restrict__ W_ih,
+            const float* __restrict__ b_ih, float* __restrict__ gi) {
+  constexpr int G3 = 3 * H, CN = G3 / 32;
+  const int LDI = I | 1;
+  const int TS = max(1, min(T, kGruXRow / I));     // steps per x chunk
+  extern __shared__ __align__(16) float sm[];
+  float* Ws = sm;                      // [3H][LDI]
+  float* xs = Ws + G3 * LDI;           // [64][TS*I]
+  const int tid = threadIdx.x, w = tid >> 5, l = tid & 31;
+  const int64_t row0 = (int64_t)blockIdx.x * kGruRows;
+  const int nrows = (int)min((int64_t)kGruRows, N - row0);
+  const int r0 = w * kGruRpw;
+  for (int i = tid; i < G3 * I; i += kGruThreads) Ws[(i / I) * LDI + i % I] = __ldg(W_ih + i);
+  float bias[CN];
+#pragma unroll
+  for (int c = 0; c < CN; ++c) bias[c] = __ldg(b_ih + l + 32 * c);
+  const float* wrow = Ws + l * LDI;
+
+  for (int t0 = 0; t0 < T; t0 += TS) {
+    const int ts = min(TS, T - t0), TSI = ts * I;
+    __syncthreads();   // the previous chunk has been read (first pass: nothing to wait for)
+    const float* xg = x + row0 * T * I + (int64_t)t0 * I;
+    for (int i = tid; i < kGruRows * TSI; i += kGruThreads) {
+      const int r = i / TSI, c = i % TSI;
+      xs[i] = r < nrows ? __ldg(xg + (int64_t)r * T * I + c) : 0.f;
+    }
+    __syncthreads();
+    for (int tt = 0; tt < ts; ++tt) {
+      float acc[kGruRpw][CN];
+#pragma unroll
+      for (int i = 0; i < kGruRpw; ++i)
+#pragma unroll
+        for (int c = 0; c < CN; ++c) acc[i][c] = bias[c];
+      const float* xr = xs + r0 * TSI + tt * I;
+      for (int k = 0; k < I; ++k) {
+        float xv[kGruRpw];
+#pragma unroll
+        for (int i = 0; i < kGruRpw; ++i) xv[i] = xr[i * TSI + k];
+#pragma unroll
+        for (int c = 0; c < CN; ++c) {
+          const float wv = wrow[32 * c * LDI + k];
+#pragma unroll
+          for (int i = 0; i < kGruRpw; ++i) acc[i][c] = fmaf(xv[i], wv, acc[i][c]);
+        }
+      }
+      float* o = gi + ((int64_t)(t0 + tt) * N + row0 + r0) * G3 + l;
+#pragma unroll
+      for (int i = 0; i < kGruRpw; ++i)
+        if (r0 + i < nrows) {
+#pragma unroll
+          for (int c = 0; c < CN; ++c) o[(int64_t)i * G3 + 32 * c] = acc[i][c];
+        }
+    }
+  }
+}
+
+// dW_ih of the projected layer 0: dW_ih [3H, I] = sum over the T*N rows of dgi[t][n][:]^T . x[n][t][:].
+// Row R of the time-major dgi is (t, n) = (R / N, R % N).  A persistent CTA (gridDim.x = tiles x panels, the panel of 8
+// input columns fastest so that the CTAs of one tile read the same dgi chunks at about the same time) walks chunks of 64
+// rows: dgi rows with 16-byte cp.async, the 8 x values of each row with 4-byte cp.async, double-buffered.  A warp owns 8
+// rows of a chunk, a lane 3H/32 gate columns x 8 inputs (72 accumulators at H = 96); the warps are combined in index
+// order, so a tile's sums are in a fixed order and the result is the same run to run.  Bound by the bytes of dgi: an
+// input wider than 8 reads dgi once per panel.
+constexpr int kGruXwChunk = 64;
+constexpr int kGruXwPanel = 8;
+
+template <int H>
+__global__ void __launch_bounds__(kGruThreads, 1)
+k_gru_xwgrad(const float* __restrict__ dgi, const float* __restrict__ x, int64_t N, int T, int I,
+             float* __restrict__ parts) {
+  constexpr int G3 = 3 * H, U3 = G3 / 32, CH = kGruXwChunk, KP = kGruXwPanel;
+  extern __shared__ __align__(16) float sm[];
+  float* Gs = sm;                      // [2][CH][3H]
+  float* Xs = sm + 2 * CH * G3;        // [2][CH][8]
+  const int P = (I + KP - 1) / KP;
+  const int tile = blockIdx.x / P, p = blockIdx.x % P, tiles = gridDim.x / P;
+  const int k0 = p * KP, kw = min(KP, I - k0);
+  const int tid = threadIdx.x, w = tid >> 5, l = tid & 31;
+  const int64_t rows = N * T, nchunks = ceil_div<int64_t>(rows, CH);
+  for (int i = tid; i < 2 * CH * KP; i += kGruThreads) Xs[i] = 0.f;   // columns >= kw stay zero
+  __syncthreads();
+
+  auto load = [&](int stage, int64_t c) {
+    const int64_t R0 = c * CH;
+    const int nr = (int)min((int64_t)CH, rows - R0);
+    float* gd = Gs + stage * CH * G3;
+    const float* gsrc = dgi + R0 * G3;
+    for (int i = tid; i < CH * G3 / 4; i += kGruThreads) {
+      if (i / (G3 / 4) < nr) cp_async16(gd + 4 * i, gsrc + 4 * i);
+      else *reinterpret_cast<float4*>(gd + 4 * i) = f4zero();
+    }
+    float* xd = Xs + stage * CH * KP;
+    for (int i = tid; i < CH * KP; i += kGruThreads) {
+      const int r = i / KP, k = i % KP;
+      if (k >= kw) continue;
+      if (r < nr) {
+        const int64_t R = R0 + r, t = R / N, n = R - t * N;
+        const unsigned d = (unsigned)__cvta_generic_to_shared(xd + i);
+        asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(d), "l"(x + (n * T + t) * I + k0 + k) : "memory");
+      } else {
+        xd[i] = 0.f;
+      }
+    }
+    cp_async_commit();
+  };
+
+  float acc[U3][KP];
+#pragma unroll
+  for (int u = 0; u < U3; ++u)
+#pragma unroll
+    for (int k = 0; k < KP; ++k) acc[u][k] = 0.f;
+  int stage = 0;
+  if (tile < nchunks) load(0, tile);
+  for (int64_t c = tile; c < nchunks; c += tiles) {
+    const int64_t nxt = c + tiles;
+    if (nxt < nchunks) { load(stage ^ 1, nxt); cp_async_wait<1>(); }
+    else cp_async_wait<0>();
+    __syncthreads();
+    const float* g = Gs + stage * CH * G3 + (w * kGruRpw) * G3 + l;
+    const float* xr = Xs + stage * CH * KP + (w * kGruRpw) * KP;
+#pragma unroll 2
+    for (int i = 0; i < kGruRpw; ++i) {
+      const float4 xa = *reinterpret_cast<const float4*>(xr + i * KP);
+      const float4 xb = *reinterpret_cast<const float4*>(xr + i * KP + 4);
+      const float xv[KP] = {xa.x, xa.y, xa.z, xa.w, xb.x, xb.y, xb.z, xb.w};
+#pragma unroll
+      for (int u = 0; u < U3; ++u) {
+        const float gv = g[i * G3 + 32 * u];
+#pragma unroll
+        for (int k = 0; k < KP; ++k) acc[u][k] = fmaf(gv, xv[k], acc[u][k]);
+      }
+    }
+    __syncthreads();
+    stage ^= 1;
+  }
+
+  // warps combined in index order: red [8 warps][U3][KP][32] fits in Gs for every supported H
+  float* red = sm;
+  float* mine = red + (w * U3 * KP) * 32 + l;
+#pragma unroll
+  for (int u = 0; u < U3; ++u)
+#pragma unroll
+    for (int k = 0; k < KP; ++k) mine[(u * KP + k) * 32] = acc[u][k];
+  __syncthreads();
+  float* out = parts + (int64_t)tile * G3 * I + k0;
+  for (int o = tid; o < G3 * kw; o += kGruThreads) {
+    const int j = o / kw, k = o % kw, u = j / 32, ln = j % 32;
+    float s = 0.f;
+#pragma unroll
+    for (int ww = 0; ww < kGruThreads / 32; ++ww) s += red[(ww * U3 * KP + u * KP + k) * 32 + ln];
+    out[(int64_t)j * I + k] = s;
+  }
+}
+
 int64_t gru_wgrad_tiles(int64_t rows) {
   return std::min<int64_t>(num_sms(), ceil_div<int64_t>(rows, kGruWgChunk));
 }
@@ -586,6 +757,11 @@ constexpr int gru_proj_rows(bool fwd) { return (kGruThreads / 32) * (fwd ? 8 : 1
 int64_t gru_proj_smem(int H, bool fwd) {
   return 4ll * (fwd ? 3ll * H * (H + 4) : (int64_t)H * (3 * H + 4)) + 4ll * 2 * gru_proj_rows(fwd) * H;
 }
+int64_t gru_xproj_smem(int H, int T, int I) {
+  const int64_t ts = std::max(1, std::min(T, kGruXRow / I));
+  return 4ll * (3ll * H * (I | 1) + (int64_t)kGruRows * ts * I);
+}
+int64_t gru_xwgrad_smem(int H) { return 4ll * 2 * kGruXwChunk * (3 * H + kGruXwPanel); }
 bool gru_hidden_ok(int32_t H) { return H == 32 || H == 64 || H == 96; }
 
 int gru_check(const char* who, int64_t N, int32_t T, int32_t I, int32_t H) {
@@ -727,10 +903,82 @@ int gru_project_impl(const char* who, const float* in, int64_t rows, int32_t H, 
   }
 }
 
+// layer 0 of the projected path: H in {32, 64, 96}, 1 <= I <= kGruMaxProjI, any T
+int gru_check_projected(const char* who, int64_t N, int32_t T, int32_t I, int32_t H) {
+  SLDM_REQUIRE(N >= 0 && T >= 1 && I >= 1, SLDM_EINVAL, "%s: bad sizes N=%lld T=%d I=%d", who, (long long)N, T, I);
+  SLDM_REQUIRE(gru_hidden_ok(H), SLDM_EUNSUPPORTED, "%s: hidden size %d (fused path: 32, 64, 96)", who, H);
+  SLDM_REQUIRE(I <= kGruMaxProjI, SLDM_EUNSUPPORTED, "%s: input width %d > %d", who, I, kGruMaxProjI);
+  SLDM_REQUIRE(ceil_div<int64_t>(N, kGruRows) < (1ll << 31), SLDM_EUNSUPPORTED, "%s: N too large", who);
+  return SLDM_OK;
+}
+
+template <int H>
+int gru_xproj_launch(const float* x, int64_t N, int T, int I, const float* W_ih, const float* b_ih, float* gi,
+                     cudaStream_t s) {
+  const int64_t smem = gru_xproj_smem(H, T, I);
+  SLDM_OPT_IN_SMEM((k_gru_xproj<H>), gru_xproj_smem(H, 1, kGruMaxProjI));
+  k_gru_xproj<H><<<(unsigned)ceil_div<int64_t>(N, kGruRows), kGruThreads, (size_t)smem, s>>>(x, N, T, I, W_ih, b_ih,
+                                                                                              gi);
+  SLDM_LAUNCH_CHECK("k_gru_xproj");
+  return SLDM_OK;
+}
+
+template <int H>
+int gru_xwgrad_launch(const float* dgi, const float* x, int64_t N, int T, int I, float* parts, cudaStream_t s) {
+  const int64_t smem = gru_xwgrad_smem(H);
+  const int64_t grid = gru_wgrad_tiles(N * (int64_t)T) * ceil_div<int64_t>(I, kGruXwPanel);
+  SLDM_OPT_IN_SMEM((k_gru_xwgrad<H>), smem);
+  k_gru_xwgrad<H><<<(unsigned)grid, kGruThreads, (size_t)smem, s>>>(dgi, x, N, T, I, parts);
+  SLDM_LAUNCH_CHECK("k_gru_xwgrad");
+  return SLDM_OK;
+}
+
 }  // namespace
 }  // namespace sldm
 
 using namespace sldm;
+
+extern "C" int sldm_gru_projected_supported(int32_t I, int32_t H) {
+  return gru_hidden_ok(H) && I >= 1 && I <= kGruMaxProjI &&
+         std::max(gru_xproj_smem(H, 1, kGruMaxProjI), gru_xwgrad_smem(H)) <= kGruSmemMax &&
+         std::max(gru_fwd_gi_smem(H), gru_bwd_smem(H, 1, 0)) <= kGruSmemMax &&
+         std::max(gru_proj_smem(H, true), gru_proj_smem(H, false)) <= kGruSmemMax;
+}
+
+extern "C" int sldm_gru_input_project_forward(const float* x, int64_t N, int32_t T, int32_t I, int32_t H,
+                                              const float* W_ih, const float* b_ih, float* gi, sldm_stream_t stream) {
+  const char* who = "sldm_gru_input_project_forward";
+  int rc = gru_check_projected(who, N, T, I, H);
+  if (rc) return rc;
+  if (N == 0) return SLDM_OK;
+  SLDM_REQUIRE(x && W_ih && b_ih && gi, SLDM_EINVAL, "%s: NULL pointer", who);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  switch (H) {
+    case 32: return gru_xproj_launch<32>(x, N, T, I, W_ih, b_ih, gi, s);
+    case 64: return gru_xproj_launch<64>(x, N, T, I, W_ih, b_ih, gi, s);
+    default: return gru_xproj_launch<96>(x, N, T, I, W_ih, b_ih, gi, s);
+  }
+}
+
+extern "C" int sldm_gru_input_wgrad(const float* dgi, const float* x, int64_t N, int32_t T, int32_t I, int32_t H,
+                                    float* partials, int64_t partial_tiles, sldm_stream_t stream) {
+  const char* who = "sldm_gru_input_wgrad";
+  int rc = gru_check_projected(who, N, T, I, H);
+  if (rc) return rc;
+  if (N == 0) return SLDM_OK;
+  SLDM_REQUIRE(dgi && x && partials, SLDM_EINVAL, "%s: NULL pointer", who);
+  const int64_t tiles = gru_wgrad_tiles(N * (int64_t)T);
+  SLDM_REQUIRE(partial_tiles >= tiles, SLDM_EWORKSPACE, "%s: %lld partial tiles < %lld", who,
+               (long long)partial_tiles, (long long)tiles);
+  SLDM_REQUIRE((reinterpret_cast<uintptr_t>(dgi) & 15u) == 0, SLDM_EINVAL, "%s: dgi must be 16-byte aligned", who);
+  SLDM_REQUIRE((reinterpret_cast<uintptr_t>(x) & 3u) == 0, SLDM_EINVAL, "%s: x must be 4-byte aligned", who);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  switch (H) {
+    case 32: return gru_xwgrad_launch<32>(dgi, x, N, T, I, partials, s);
+    case 64: return gru_xwgrad_launch<64>(dgi, x, N, T, I, partials, s);
+    default: return gru_xwgrad_launch<96>(dgi, x, N, T, I, partials, s);
+  }
+}
 
 extern "C" int sldm_gru_supported(int32_t T, int32_t I, int32_t H) {
   return gru_hidden_ok(H) && T >= 1 && I >= 1 && I <= kGruMaxI &&

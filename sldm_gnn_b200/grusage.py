@@ -22,7 +22,8 @@ import os
 import torch
 import torch.nn as nn
 
-from .gru import fused_gru_eligible, fused_gru_stack_eligible, gru_last_hidden, gru_stack_last_hidden
+from .gru import (fused_gru_eligible, fused_gru_projected_eligible, fused_gru_stack_eligible, gru_last_hidden,
+                  gru_projected_last_hidden, gru_stack_last_hidden)
 from .map_attention import MapSpatialAttention
 from .ops import index_checks
 from .readout import global_max_pool, global_mean_max_pool, global_mean_pool
@@ -161,7 +162,11 @@ class GruSage(nn.Module):
         configuration (main.py:42-44: hidden 96, one layer, 6 dynamic features).  A stacked head (gru_num_layers > 1)
         with the same limits on its first layer runs on the same kernels layer by layer (gru_stack_last_hidden: the
         layers above take their input projection from k_gru_proj and have no limit on T), unless inter-layer dropout
-        is active in training.  Anything else, or SLDM_DISABLE_FUSED_GRU=1, goes through torch's library GRU, and there through ATen's native path (one cuBLAS
+        is active in training.  Sequences too long or inputs too wide for layer 0's x tile (for example more than 30
+        frames at hidden 96, or more than 8 dynamic features) take the projected path (gru_projected_last_hidden: x is
+        first projected into the gate pre-activations gi by k_gru_xproj, up to 128 features, any number of frames).
+        The tile is preferred wherever it applies, since it saves gi's round trip through HBM; the choice follows from
+        the shape alone.  Anything else, or SLDM_DISABLE_FUSED_GRU=1, goes through torch's library GRU, and there through ATen's native path (one cuBLAS
         GEMM + one fused cell kernel per step) rather than cuDNN's: measured on B200 at the C2 shape (205 k sequences
         x 16 frames, input 6, hidden 96) the native path takes 35 ms forward + backward against 118 ms, and it computes
         in true fp32 -- cuDNN's RNN runs TF32 under torch's default flags (2e-4 off the CPU result,
@@ -173,6 +178,8 @@ class GruSage(nn.Module):
                 return gru_last_hidden(self.gru, x)
             if fused_gru_stack_eligible(self.gru, x):
                 return gru_stack_last_hidden(self.gru, x)
+            if fused_gru_projected_eligible(self.gru, x):
+                return gru_projected_last_hidden(self.gru, x)
         n, per_seq = x.size(0), x.size(1) * 3 * self.gru.hidden_size
         rows = max(1, (1 << 30) // max(per_seq, 1))
         with torch.backends.cudnn.flags(enabled=False):
