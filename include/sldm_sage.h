@@ -277,7 +277,10 @@ int sldm_collate_graph_index(const void* table_dev, const int64_t* node_ptr_dev,
  * forward also returns idx [B,K] int64 (ascending distance), dist [B,K], w [B,K] (the saved tensors of backward).
  * backward: gradients for emb (demb [S,D], may be NULL) and the four MLP tensors; positions and centroids are data.
  * csr = membership CSR of idx: sldm_csr_build_pairs(NULL, idx, B*K, csr_nodes >= S, ...) (only needed for demb).
- * K <= 8, H <= 64, S >= K (else SLDM_ESHAPE, like torch.topk).
+ * K <= 32 (sldm_map_attention_max_k()), H <= 64, S >= K (else SLDM_ESHAPE, like torch.topk).  K <= 8 and K > 8 run
+ * different kernels (a per-thread sorted list up to 8, one warp per position above) under the same contract.
+ * Backward workspace: sldm_map_attention_workspace_bytes_k(B, H, K); sldm_map_attention_workspace_bytes(B, H) is the
+ * same size for any K <= 8.  K > 8 also needs B * K < 2^31 - 2^20 (the membership CSR).
  * Two forward entry points with identical results (bit for bit):
  *   sldm_map_attention_forward       exhaustive scan of the S centroids per position (no preparation);
  *   sldm_map_attention_forward_grid  ring search over a uniform grid of the centroids.  The centroids are a constant
@@ -287,6 +290,8 @@ int sldm_collate_graph_index(const void* table_dev, const int64_t* node_ptr_dev,
  * Non-finite positions or centroids: memory-safe, selection unspecified.
  */
 int64_t sldm_map_attention_workspace_bytes(int64_t B, int32_t H);
+int64_t sldm_map_attention_workspace_bytes_k(int64_t B, int32_t H, int32_t K);
+int     sldm_map_attention_max_k(void);
 int64_t sldm_map_grid_bytes(int64_t S);
 int     sldm_map_grid_build(const float* centroids, int64_t S, void* grid, int64_t grid_bytes, sldm_stream_t stream);
 int     sldm_map_attention_forward_grid(const float* pos, int64_t B, const void* grid, int64_t grid_bytes, int64_t S,

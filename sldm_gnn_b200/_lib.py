@@ -68,6 +68,8 @@ _PROTOS = {
     "sldm_concat_chunks": (C.c_int, [_p, _i64, _i64, _p, _p]),
     "sldm_collate_graph_index": (C.c_int, [_p, _p, _i64, _i64, _i64, _i64, _p, _p, _p]),
     "sldm_map_attention_workspace_bytes": (_i64, [_i64, _i32]),
+    "sldm_map_attention_workspace_bytes_k": (_i64, [_i64, _i32, _i32]),
+    "sldm_map_attention_max_k": (C.c_int, []),
     "sldm_map_attention_forward": (C.c_int, [_p, _i64, _p, _i64, _p, _i32, _i32, _p, _p, _p, _p, _i32, _p, _p, _p, _p, _p]),
     "sldm_map_grid_bytes": (_i64, [_i64]),
     "sldm_map_grid_build": (C.c_int, [_p, _i64, _p, _i64, _p]),

@@ -693,7 +693,339 @@ k_map_attention_reduce(const float* __restrict__ part, int nparts, int H, float*
   }
 }
 
-// kernel for the MLP gradients: elements = B * kMaK at most; the partial count is fixed by B alone (workspace sizing)
+// ------------------------------------------------------------------------------------------------------ K > 8 --
+// The kernels above keep K-long arrays per thread: the grid search a sorted list of K 64-bit keys (48 registers at K = 8,
+// the cap of its __launch_bounds__(256, 5)), k_map_attention_bwd_ds K embedding rows in flight (116 registers at K = 8).
+// A 32-key list alone would take 64 registers.  For 8 < K <= 32 every kernel below works with one WARP per vehicle and
+// the warp's K best (distance, index) keys in lanes 0..K-1, the structure of k_map_attention_fwd.  Same keys, same
+// distance arithmetic, same tie rule: the selected set is exactly the K nearest, whatever the visit order.
+constexpr int kMaKWide = 32;
+constexpr int64_t kMaCsrMax = ((int64_t)1 << 31) - ((int64_t)1 << 20);   // pairs of the int32 membership CSR
+
+// Offers one candidate (squared distance c2, segment ci; both warp-uniform) to the warp's ascending list L (lanes
+// 0..K-1) with a warp-uniform shift: a lane keeps its key if it is smaller, else takes the candidate (lane 0, or the left
+// neighbour's key is smaller) or the left neighbour's key.  Then the filter is tightened to the new K-th best, inflated
+// by a few ulp so that a candidate that would TIE after the rounding of sqrt still gets in.  NaN passes the filter: the
+// exact key comparison decides, and a vehicle whose distances are all NaN still fills its list with valid indices.
+__device__ __forceinline__ void ma_offer(unsigned long long& L, float& thr2, float c2, int ci, int lane, int K) {
+  if (c2 > thr2) return;                           // the threshold may have tightened inside this round (uniform)
+  const unsigned long long key = pack_key(__fsqrt_rn(c2), ci);
+  const bool lt = L < key;
+  const unsigned long long prev = __shfl_up_sync(0xffffffffu, L, 1);
+  const int prevlt = __shfl_up_sync(0xffffffffu, (int)lt, 1);
+  if (lane < K) L = lt ? L : ((lane == 0 || prevlt) ? key : prev);
+  const unsigned long long worst = __shfl_sync(0xffffffffu, L, K - 1);
+  if (worst != ~0ull) {
+    const float wd = __uint_as_float((unsigned)(worst >> 32));
+    thr2 = __fmul_rn(__fmul_rn(wd, wd), 1.000001f);
+  }
+}
+
+// One round of up to 32 candidates, lane i holding (d2, ci) when `has`: a ballot against the threshold picks the few
+// that can enter, and they are offered in lane order.
+__device__ __forceinline__ void ma_round(unsigned long long& L, float& thr2, bool has, float d2, int ci, int lane, int K) {
+  unsigned m = __ballot_sync(0xffffffffu, has && !(d2 > thr2));
+  while (m) {
+    const int src = __ffs(m) - 1;
+    m &= m - 1;
+    ma_offer(L, thr2, __shfl_sync(0xffffffffu, d2, src), __shfl_sync(0xffffffffu, ci, src), lane, K);
+  }
+}
+
+// dx*dx + dy*dy without FMA contraction: the same operations torch.norm performs
+__device__ __forceinline__ float ma_d2(float px, float py, float cx, float cy) {
+  const float dx = __fsub_rn(px, cx), dy = __fsub_rn(py, cy);
+  return __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
+}
+
+// The epilogue of both K > 8 forward kernels, so that they return the same bits: the score MLP on lanes 0..K-1, the
+// softmax max and denominator by the 32-lane butterfly, w = ex / den (IEEE), the saved tensors, then
+// ctx = sum_k w_k emb[idx_k] as one FMA chain in ascending k, lane = column.  The (weight, row) pairs are broadcast through
+// the warp's 32 slots of shared memory.  Called by the whole warp.
+__device__ __forceinline__ void ma_wide_epilogue(unsigned long long L, int lane, int K, int64_t b,
+                                                 const float* s_w1, const float* s_b1, const float* s_w2, int H,
+                                                 const float* __restrict__ b2, const float* __restrict__ emb, int D,
+                                                 float* s_wt, int* s_ix, float* __restrict__ ctx, int64_t* __restrict__ idx_out,
+                                                 float* __restrict__ dist_out, float* __restrict__ w_out) {
+  const float kd = __uint_as_float((unsigned)(L >> 32));          // lane k (< K): the k-th nearest
+  const int kidx = (int)(unsigned)(L & 0xffffffffu);
+  float score = -INFINITY;
+  if (lane < K) {
+    float acc = 0.f;
+    for (int h = 0; h < H; ++h) {
+      const float pre = fmaf(s_w1[h], kd, s_b1[h]);
+      acc = fmaf(s_w2[h], pre > 0.f ? pre : 0.f, acc);
+    }
+    score = acc + __ldg(b2);
+  }
+  float mx = score;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  const float ex = lane < K ? expf(score - mx) : 0.f;
+  float den = ex;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) den += __shfl_xor_sync(0xffffffffu, den, o);
+  const float w = __fdiv_rn(ex, den);
+  if (lane < K) {
+    idx_out[b * K + lane] = kidx;
+    dist_out[b * K + lane] = kd;
+    w_out[b * K + lane] = w;
+    s_wt[lane] = w;
+    s_ix[lane] = kidx;
+  }
+  __syncwarp();
+  if (D == 32) {
+    float acc = 0.f;
+#pragma unroll 8
+    for (int k = 0; k < K; ++k) acc = fmaf(s_wt[k], __ldg(emb + (int64_t)s_ix[k] * 32 + lane), acc);
+    ctx[b * 32 + lane] = acc;
+  } else {
+    for (int c = lane; c < D; c += 32) {
+      float acc = 0.f;
+#pragma unroll 8
+      for (int k = 0; k < K; ++k) acc = fmaf(s_wt[k], __ldg(emb + (int64_t)s_ix[k] * D + c), acc);
+      ctx[b * D + c] = acc;
+    }
+  }
+  __syncwarp();                                    // the slots are rewritten by the warp's next vehicle
+}
+
+// Exhaustive scan for K > 8: k_map_attention_fwd with a runtime K and the shared insertion and epilogue.
+__global__ void __launch_bounds__(256)
+k_map_attention_fwd_wide(const float* __restrict__ pos, int64_t B, const float2* __restrict__ cent, int S,
+                         const float* __restrict__ emb, int D, const float* __restrict__ W1, const float* __restrict__ b1,
+                         const float* __restrict__ W2, const float* __restrict__ b2, int H, int K,
+                         float* __restrict__ ctx, int64_t* __restrict__ idx_out, float* __restrict__ dist_out,
+                         float* __restrict__ w_out) {
+  __shared__ float2 s_c[kMaTile];
+  __shared__ float s_w1[kMaH], s_b1[kMaH], s_w2[kMaH];
+  __shared__ float s_wt[8][32];
+  __shared__ int s_ix[8][32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int h = threadIdx.x; h < H; h += 256) { s_w1[h] = W1[h]; s_b1[h] = b1[h]; s_w2[h] = W2[h]; }
+  const bool single = S <= kMaTile;
+  if (single) {
+    for (int i = threadIdx.x; i < S; i += 256) s_c[i] = __ldg(cent + i);
+  }
+  __syncthreads();
+  for (int64_t vb = blockIdx.x; vb * 8 < B; vb += gridDim.x) {
+    const int64_t b = vb * 8 + warp;
+    const bool live = b < B;                       // warp-uniform
+    const float px = live ? __ldg(pos + 2 * b) : 0.f, py = live ? __ldg(pos + 2 * b + 1) : 0.f;
+    unsigned long long L = ~0ull;
+    float thr2 = INFINITY;
+    for (int t0 = 0; t0 < S; t0 += kMaTile) {
+      const int tn = min(kMaTile, S - t0);
+      if (!single) {
+        __syncthreads();
+        for (int i = threadIdx.x; i < tn; i += 256) s_c[i] = __ldg(cent + t0 + i);
+        __syncthreads();
+      }
+      if (live) {
+        int i0 = 0;
+        if (t0 == 0) {
+          // bootstrap: the first 32 segments sorted by a warp bitonic network; S >= K, so lanes 0..K-1 get real keys
+          unsigned long long key = ~0ull;
+          if (lane < tn) key = pack_key(__fsqrt_rn(ma_d2(px, py, s_c[lane].x, s_c[lane].y)), lane);
+#pragma unroll
+          for (int k = 2; k <= 32; k <<= 1) {
+#pragma unroll
+            for (int j = k >> 1; j > 0; j >>= 1) {
+              const unsigned long long other = __shfl_xor_sync(0xffffffffu, key, j);
+              const bool take_min = ((lane & k) == 0) == ((lane & j) == 0);
+              key = (take_min == (other < key)) ? other : key;
+            }
+          }
+          L = lane < K ? key : ~0ull;
+          const float wd = __uint_as_float((unsigned)(__shfl_sync(0xffffffffu, L, K - 1) >> 32));
+          thr2 = __fmul_rn(__fmul_rn(wd, wd), 1.000001f);
+          i0 = 32;
+        }
+        for (; i0 < tn; i0 += 32) {
+          const int i = i0 + lane;
+          const bool has = i < tn;
+          ma_round(L, thr2, has, has ? ma_d2(px, py, s_c[i].x, s_c[i].y) : INFINITY, t0 + i, lane, K);
+        }
+      }
+    }
+    if (live) ma_wide_epilogue(L, lane, K, b, s_w1, s_b1, s_w2, H, b2, emb, D, s_wt[warp], s_ix[warp], ctx, idx_out, dist_out, w_out);
+  }
+}
+
+// Grid search for K > 8, one warp per vehicle: the cells of k_map_attention_grid_fwd in the same order (the 3 x 3 block
+// around the own cell, then square rings) and the same stopping rule; a run of entries is taken 32 at a time, one per lane.
+__global__ void __launch_bounds__(256)
+k_map_attention_grid_fwd_wide(const float* __restrict__ pos, int64_t B, const MapGridHeader* __restrict__ hdr,
+                              const int* __restrict__ cell_start, const float4* __restrict__ entries,
+                              const float* __restrict__ emb, int D, const float* __restrict__ W1, const float* __restrict__ b1,
+                              const float* __restrict__ W2, const float* __restrict__ b2, int H, int K,
+                              float* __restrict__ ctx, int64_t* __restrict__ idx_out, float* __restrict__ dist_out,
+                              float* __restrict__ w_out) {
+  __shared__ float s_w1[kMaH], s_b1[kMaH], s_w2[kMaH];
+  __shared__ float s_wt[8][32];
+  __shared__ int s_ix[8][32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int h = threadIdx.x; h < H; h += 256) { s_w1[h] = W1[h]; s_b1[h] = b1[h]; s_w2[h] = W2[h]; }
+  __syncthreads();
+  const int64_t b = (int64_t)blockIdx.x * 8 + warp;
+  if (b >= B) return;                              // warp-uniform; no block barrier follows
+  const float px = __ldg(pos + 2 * b), py = __ldg(pos + 2 * b + 1);
+  const float minx = __ldg(&hdr->minx), miny = __ldg(&hdr->miny), wx = __ldg(&hdr->wx), wy = __ldg(&hdr->wy);
+  const float slack = __ldg(&hdr->slack);
+  const int G = __ldg(&hdr->G);
+  const int cx = grid_coord(px, minx, __ldg(&hdr->inv_wx), G), cy = grid_coord(py, miny, __ldg(&hdr->inv_wy), G);
+  unsigned long long L = ~0ull;
+  float thr2 = INFINITY;
+  auto scan = [&](int beg, int end) {
+    for (int e0 = beg; e0 < end; e0 += 32) {
+      const int e = e0 + lane;
+      const bool has = e < end;
+      float d2 = INFINITY;
+      int ci = 0;
+      if (has) {
+        const float4 c = __ldg(entries + e);
+        d2 = ma_d2(px, py, c.x, c.y);
+        ci = __float_as_int(c.z);
+      }
+      ma_round(L, thr2, has, d2, ci, lane, K);
+    }
+  };
+  {
+    const int xa = max(cx - 1, 0), xb = min(cx + 1, G - 1);
+    for (int y = max(cy - 1, 0); y <= min(cy + 1, G - 1); ++y)
+      scan(__ldg(cell_start + y * G + xa), __ldg(cell_start + y * G + xb + 1));
+  }
+  for (int r = 1;; ++r) {
+    const int x0 = cx - r, x1 = cx + r, y0 = cy - r, y1 = cy + r;
+    if (r > 1) {
+      const int xa = max(x0, 0), xb = min(x1, G - 1);
+      if (y0 >= 0) scan(__ldg(cell_start + y0 * G + xa), __ldg(cell_start + y0 * G + xb + 1));
+      if (y1 <= G - 1) scan(__ldg(cell_start + y1 * G + xa), __ldg(cell_start + y1 * G + xb + 1));
+      for (int y = max(y0 + 1, 0); y <= min(y1 - 1, G - 1); ++y) {
+        if (x0 >= 0) scan(__ldg(cell_start + y * G + x0), __ldg(cell_start + y * G + x0 + 1));
+        if (x1 <= G - 1) scan(__ldg(cell_start + y * G + x1), __ldg(cell_start + y * G + x1 + 1));
+      }
+    }
+    float bound = INFINITY;
+    bool more = false;
+    if (x0 > 0) { more = true; bound = fminf(bound, px - (minx + (float)x0 * wx)); }
+    if (x1 < G - 1) { more = true; bound = fminf(bound, (minx + (float)(x1 + 1) * wx) - px); }
+    if (y0 > 0) { more = true; bound = fminf(bound, py - (miny + (float)y0 * wy)); }
+    if (y1 < G - 1) { more = true; bound = fminf(bound, (miny + (float)(y1 + 1) * wy) - py); }
+    if (!more) break;                              // the whole grid has been visited
+    const unsigned long long worst = __shfl_sync(0xffffffffu, L, K - 1);
+    if (worst != ~0ull && __uint_as_float((unsigned)(worst >> 32)) < bound - slack) break;
+  }
+  ma_wide_epilogue(L, lane, K, b, s_w1, s_b1, s_w2, H, b2, emb, D, s_wt[warp], s_ix[warp], ctx, idx_out, dist_out, w_out);
+}
+
+// ds for K > 8, one warp per vehicle, lane = neighbour k: gw_k = <emb[idx_k], dctx_b> streams the lane's own embedding
+// row (16-byte loads when VEC), sum_j w_j gw_j by the 32-lane butterfly (fixed order), ds_k = w_k (gw_k - sum_j w_j gw_j).
+template <bool VEC>
+__global__ void __launch_bounds__(256)
+k_map_attention_bwd_ds_wide(const float* __restrict__ dctx, int64_t B, const float* __restrict__ emb, int D, int K,
+                            const int64_t* __restrict__ idx, const float* __restrict__ wgt, float* __restrict__ ds_out) {
+  const int lane = threadIdx.x & 31;
+  const int64_t b = ((int64_t)blockIdx.x * 256 + threadIdx.x) >> 5;
+  if (b >= B) return;                              // warp-uniform
+  const bool on = lane < K;
+  const float wk = on ? __ldg(wgt + b * K + lane) : 0.f;
+  float gw = 0.f;
+  if (on) {
+    const float* row = emb + __ldg(idx + b * K + lane) * (int64_t)D;
+    const float* g = dctx + b * D;
+    if constexpr (VEC) {
+#pragma unroll 4
+      for (int c = 0; c < D; c += 4) {
+        const float4 e = __ldg(reinterpret_cast<const float4*>(row + c));
+        const float4 x = __ldg(reinterpret_cast<const float4*>(g + c));
+        gw = fmaf(e.w, x.w, fmaf(e.z, x.z, fmaf(e.y, x.y, fmaf(e.x, x.x, gw))));
+      }
+    } else {
+#pragma unroll 4
+      for (int c = 0; c < D; ++c) gw = fmaf(__ldg(row + c), __ldg(g + c), gw);
+    }
+  }
+  float dot = wk * gw;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, o);
+  if (on) ds_out[b * K + lane] = wk * (gw - dot);
+}
+
+// The MLP gradients for K > 8: lanes and partials as in k_map_attention_bwd_mlp, but every lane reads its vehicle's K
+// (dist, ds) pairs itself (the HL lanes of a vehicle slot read the same words).  The K terms of a vehicle are still summed
+// locally before they enter the running sums (they cancel: sum_k ds_k = 0).
+__global__ void __launch_bounds__(256)
+k_map_attention_bwd_mlp_wide(const float* __restrict__ dist, const float* __restrict__ ds, int64_t B, int K, int64_t per_cta,
+                             const float* __restrict__ W1, const float* __restrict__ b1, const float* __restrict__ W2,
+                             int H, int HL, float* __restrict__ part) {
+  __shared__ float s_p[8][3 * kMaH + 1];
+  __shared__ float s_g[8][32][7];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int EG = 32 / HL, hl = lane % HL, eg = lane / HL;
+  float w1[2], bb[2], w2[2];
+#pragma unroll
+  for (int q = 0; q < 2; ++q) {
+    const int h = hl + 32 * q;
+    const bool on = h < H && (q == 0 || HL == 32);
+    w1[q] = on ? __ldg(W1 + h) : 0.f; bb[q] = on ? __ldg(b1 + h) : 0.f; w2[q] = on ? __ldg(W2 + h) : 0.f;
+  }
+  float a1[2] = {0.f, 0.f}, a2[2] = {0.f, 0.f}, a3[2] = {0.f, 0.f}, a4 = 0.f;
+  const int64_t beg = (int64_t)blockIdx.x * per_cta, end = min(B, beg + per_cta);
+  for (int64_t v = beg + warp * EG + eg; v < end; v += 8 * EG) {
+    float l1[2] = {0.f, 0.f}, l2[2] = {0.f, 0.f}, l3[2] = {0.f, 0.f}, l4 = 0.f;
+    for (int k = 0; k < K; ++k) {
+      const float d = __ldg(dist + v * K + k), g = __ldg(ds + v * K + k);
+      l4 += g;
+#pragma unroll
+      for (int q = 0; q < 2; ++q) {
+        if (q == 1 && HL < 32) break;
+        const float pre = fmaf(w1[q], d, bb[q]);
+        const bool pos = pre > 0.f;
+        l3[q] = fmaf(g, pos ? pre : 0.f, l3[q]);
+        const float da = pos ? g * w2[q] : 0.f;
+        l1[q] = fmaf(da, d, l1[q]);
+        l2[q] += da;
+      }
+    }
+    a4 += l4;
+#pragma unroll
+    for (int q = 0; q < 2; ++q) { a1[q] += l1[q]; a2[q] += l2[q]; a3[q] += l3[q]; }
+  }
+  // combine the vehicle slots of a warp in slot order, then the warps in warp order
+  s_g[warp][lane][0] = a1[0]; s_g[warp][lane][1] = a1[1]; s_g[warp][lane][2] = a2[0]; s_g[warp][lane][3] = a2[1];
+  s_g[warp][lane][4] = a3[0]; s_g[warp][lane][5] = a3[1]; s_g[warp][lane][6] = a4;
+  __syncwarp();
+  if (lane < HL) {
+    float t[7] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    for (int e = 0; e < EG; ++e)
+#pragma unroll
+      for (int v = 0; v < 7; ++v) t[v] += s_g[warp][e * HL + lane][v];
+#pragma unroll
+    for (int q = 0; q < 2; ++q) {
+      const int h = lane + 32 * q;
+      if (h < H && (q == 0 || HL == 32)) { s_p[warp][h] = t[q]; s_p[warp][H + h] = t[2 + q]; s_p[warp][2 * H + h] = t[4 + q]; }
+    }
+    if (lane == 0) s_p[warp][3 * H] = t[6];
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < 3 * H + 1; i += 256) {
+    float s = 0.f;
+#pragma unroll
+    for (int w = 0; w < 8; ++w) s += s_p[w][i];
+    part[(int64_t)blockIdx.x * (3 * H + 1) + i] = s;
+  }
+}
+
+// k_map_attention_demb for K = 9..32: one instance per K (K only divides the member position)
+template <int KK>
+static void launch_demb_wide(int K, unsigned S, size_t smb, cudaStream_t s, const float* dctx, int D, const float* w,
+                             const int32_t* rp, const int32_t* mem, float* demb) {
+  if (K == KK) k_map_attention_demb<KK><<<S, 32 * kDembWarps, smb, s>>>(dctx, D, w, rp, mem, demb);
+  else if constexpr (KK < kMaKWide) launch_demb_wide<KK + 1>(K, S, smb, s, dctx, D, w, rp, mem, demb);
+}
+
+// kernel for the MLP gradients: the partial count is fixed by B alone (workspace sizing)
 static int mlp_grid(int64_t B) { return (int)std::max<int64_t>(1, std::min<int64_t>(ceil_div<int64_t>(B, 256), (int64_t)num_sms() * 4)); }
 
 }  // namespace sldm
@@ -706,13 +1038,21 @@ extern "C" int64_t sldm_map_attention_workspace_bytes(int64_t B, int32_t H) {
   return align_bytes(B * kMaK * 4) + align_bytes((int64_t)mlp_grid(B) * (3 * H + 1) * 4);
 }
 
+// the same layout with B * max(K, 8) floats for ds: equal to the query above for K <= 8
+extern "C" int64_t sldm_map_attention_workspace_bytes_k(int64_t B, int32_t H, int32_t K) {
+  if (B < 0 || H < 0 || K < 1 || K > kMaKWide) return -1;
+  return align_bytes(B * std::max<int64_t>(K, kMaK) * 4) + align_bytes((int64_t)mlp_grid(B) * (3 * H + 1) * 4);
+}
+
+extern "C" int sldm_map_attention_max_k(void) { return kMaKWide; }
+
 extern "C" int sldm_map_attention_forward(const float* pos, int64_t B, const float* centroids, int64_t S,
                                           const float* emb, int32_t D, int32_t K,
                                           const float* W1, const float* b1, const float* W2, const float* b2, int32_t H,
                                           float* ctx, int64_t* idx_out, float* dist_out, float* w_out,
                                           sldm_stream_t stream) {
   SLDM_REQUIRE(B >= 0 && S >= 0 && D >= 1, SLDM_EINVAL, "sldm_map_attention_forward: bad sizes");
-  SLDM_REQUIRE(K >= 1 && K <= kMaK, SLDM_EUNSUPPORTED, "sldm_map_attention_forward: k_neighbors=%d outside 1..%d", K, kMaK);
+  SLDM_REQUIRE(K >= 1 && K <= kMaKWide, SLDM_EUNSUPPORTED, "sldm_map_attention_forward: k_neighbors=%d outside 1..%d", K, kMaKWide);
   SLDM_REQUIRE(H >= 1 && H <= kMaH, SLDM_EUNSUPPORTED, "sldm_map_attention_forward: MLP width %d outside 1..%d", H, kMaH);
   SLDM_REQUIRE(S >= K, SLDM_ESHAPE, "selected index k out of range");   // torch.topk's message
   SLDM_REQUIRE(S < ((int64_t)1 << 31), SLDM_EUNSUPPORTED, "sldm_map_attention_forward: S too large");
@@ -723,6 +1063,11 @@ extern "C" int sldm_map_attention_forward(const float* pos, int64_t B, const flo
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const unsigned grid = (unsigned)std::min<int64_t>(ceil_div<int64_t>(B, 8), (int64_t)num_sms() * 8);
   const float2* c2 = reinterpret_cast<const float2*>(centroids);
+  if (K > kMaK) {
+    k_map_attention_fwd_wide<<<grid, 256, 0, s>>>(pos, B, c2, (int)S, emb, D, W1, b1, W2, b2, H, K, ctx, idx_out, dist_out, w_out);
+    SLDM_LAUNCH_CHECK("k_map_attention_fwd_wide");
+    return SLDM_OK;
+  }
 #define SLDM_MA(KK) k_map_attention_fwd<KK><<<grid, 256, 0, s>>>(pos, B, c2, (int)S, emb, D, W1, b1, W2, b2, H, ctx, idx_out, dist_out, w_out)
   switch (K) {
     case 1: SLDM_MA(1); break; case 2: SLDM_MA(2); break; case 3: SLDM_MA(3); break; case 4: SLDM_MA(4); break;
@@ -759,7 +1104,7 @@ extern "C" int sldm_map_attention_forward_grid(const float* pos, int64_t B, cons
                                                float* ctx, int64_t* idx_out, float* dist_out, float* w_out,
                                                sldm_stream_t stream) {
   SLDM_REQUIRE(B >= 0 && S >= 0 && D >= 1, SLDM_EINVAL, "sldm_map_attention_forward_grid: bad sizes");
-  SLDM_REQUIRE(K >= 1 && K <= kMaK, SLDM_EUNSUPPORTED, "sldm_map_attention_forward_grid: k_neighbors=%d outside 1..%d", K, kMaK);
+  SLDM_REQUIRE(K >= 1 && K <= kMaKWide, SLDM_EUNSUPPORTED, "sldm_map_attention_forward_grid: k_neighbors=%d outside 1..%d", K, kMaKWide);
   SLDM_REQUIRE(H >= 1 && H <= kMaH, SLDM_EUNSUPPORTED, "sldm_map_attention_forward_grid: MLP width %d outside 1..%d", H, kMaH);
   SLDM_REQUIRE(S >= K, SLDM_ESHAPE, "selected index k out of range");   // torch.topk's message
   SLDM_REQUIRE(S * (int64_t)D < ((int64_t)1 << 32), SLDM_EUNSUPPORTED, "sldm_map_attention_forward_grid: S * D must stay below 2^32");
@@ -770,6 +1115,13 @@ extern "C" int sldm_map_attention_forward_grid(const float* pos, int64_t B, cons
                "sldm_map_attention_forward_grid: NULL pointer");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const uint8_t* g = static_cast<const uint8_t*>(grid);
+  if (K > kMaK) {
+    k_map_attention_grid_fwd_wide<<<(unsigned)ceil_div<int64_t>(B, 8), 256, 0, s>>>(
+        pos, B, reinterpret_cast<const MapGridHeader*>(g), reinterpret_cast<const int*>(g + L.off_start),
+        reinterpret_cast<const float4*>(g + L.off_entries), emb, D, W1, b1, W2, b2, H, K, ctx, idx_out, dist_out, w_out);
+    SLDM_LAUNCH_CHECK("k_map_attention_grid_fwd_wide");
+    return SLDM_OK;
+  }
   const unsigned nblk = (unsigned)ceil_div<int64_t>(B, 256);
 #define SLDM_MG(KK) k_map_attention_grid_fwd<KK><<<nblk, 256, 0, s>>>(pos, B, reinterpret_cast<const MapGridHeader*>(g), \
       reinterpret_cast<const int*>(g + L.off_start), reinterpret_cast<const float4*>(g + L.off_entries), emb, D, W1, b1, W2, b2, H, \
@@ -793,7 +1145,9 @@ extern "C" int sldm_map_attention_backward(const float* dctx, int64_t B, const f
   SLDM_REQUIRE(B >= 0 && S >= 0 && D >= 1 && D <= 1024, SLDM_EINVAL, "sldm_map_attention_backward: bad sizes");
   SLDM_REQUIRE(S * (int64_t)D < ((int64_t)1 << 32) && B * (int64_t)D < ((int64_t)1 << 32), SLDM_EUNSUPPORTED,
                "sldm_map_attention_backward: S * D and B * D must stay below 2^32");
-  SLDM_REQUIRE(K >= 1 && K <= kMaK && H >= 1 && H <= kMaH, SLDM_EUNSUPPORTED, "sldm_map_attention_backward: K / H out of range");
+  SLDM_REQUIRE(K >= 1 && K <= kMaKWide && H >= 1 && H <= kMaH, SLDM_EUNSUPPORTED, "sldm_map_attention_backward: K / H out of range");
+  SLDM_REQUIRE(K <= kMaK || B * K < kMaCsrMax, SLDM_EUNSUPPORTED,
+               "sldm_map_attention_backward: B * K = %lld exceeds the int32 membership CSR", (long long)(B * K));
   SLDM_REQUIRE(dW1 && db1 && dW2 && db2, SLDM_EINVAL, "sldm_map_attention_backward: NULL gradient output");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (B == 0) {
@@ -803,10 +1157,10 @@ extern "C" int sldm_map_attention_backward(const float* dctx, int64_t B, const f
     return SLDM_OK;
   }
   SLDM_REQUIRE(dctx && emb && idx && dist && w && W1 && b1 && W2, SLDM_EINVAL, "sldm_map_attention_backward: NULL pointer");
-  SLDM_REQUIRE(workspace != nullptr && workspace_bytes >= sldm_map_attention_workspace_bytes(B, H), SLDM_EWORKSPACE,
+  SLDM_REQUIRE(workspace != nullptr && workspace_bytes >= sldm_map_attention_workspace_bytes_k(B, H, K), SLDM_EWORKSPACE,
                "sldm_map_attention_backward: workspace too small");
   float* const ds = static_cast<float*>(workspace);
-  float* const part = reinterpret_cast<float*>(static_cast<uint8_t*>(workspace) + align_bytes(B * kMaK * 4));
+  float* const part = reinterpret_cast<float*>(static_cast<uint8_t*>(workspace) + align_bytes(B * std::max(K, kMaK) * 4));
   const bool vec = (D % 4 == 0) && ((reinterpret_cast<uintptr_t>(dctx) | reinterpret_cast<uintptr_t>(emb)) & 15u) == 0;
   // persistent grid: exactly the CTAs that are resident at once (the loop prefetches across iterations)
   auto ds_grid = [&](auto kernel, int vpw) {
@@ -814,20 +1168,29 @@ extern "C" int sldm_map_attention_backward(const float* dctx, int64_t B, const f
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, 256, 0);
     return (int)std::max<int64_t>(1, std::min<int64_t>(ceil_div<int64_t>(B, 8 * vpw), (int64_t)num_sms() * std::max(per_sm, 1)));
   };
-#define SLDM_MB(KK) do { if (vec) k_map_attention_bwd_ds<KK, 8><<<ds_grid(k_map_attention_bwd_ds<KK, 8>, 4), 256, 0, s>>>(dctx, B, emb, D, idx, w, ds); \
-                         else k_map_attention_bwd_ds<KK, 32><<<ds_grid(k_map_attention_bwd_ds<KK, 32>, 1), 256, 0, s>>>(dctx, B, emb, D, idx, w, ds); } while (0)
-  switch (K) {
-    case 1: SLDM_MB(1); break; case 2: SLDM_MB(2); break; case 3: SLDM_MB(3); break; case 4: SLDM_MB(4); break;
-    case 5: SLDM_MB(5); break; case 6: SLDM_MB(6); break; case 7: SLDM_MB(7); break; default: SLDM_MB(8); break;
-  }
-#undef SLDM_MB
-  SLDM_LAUNCH_CHECK("k_map_attention_bwd_ds");
   const int mgrid = mlp_grid(B);
   const int64_t per_cta = round_up<int64_t>(ceil_div<int64_t>(B, mgrid), 256);   // vehicles per CTA
   int HL = 1;
   while (HL < H && HL < 32) HL <<= 1;              // lanes across the hidden units
-  k_map_attention_bwd_mlp<<<mgrid, 256, 0, s>>>(dist, ds, B, K, per_cta, W1, b1, W2, H, HL, part);
-  SLDM_LAUNCH_CHECK("k_map_attention_bwd_mlp");
+  if (K > kMaK) {
+    const unsigned nblk = (unsigned)ceil_div<int64_t>(B, 8);
+    if (vec) k_map_attention_bwd_ds_wide<true><<<nblk, 256, 0, s>>>(dctx, B, emb, D, K, idx, w, ds);
+    else k_map_attention_bwd_ds_wide<false><<<nblk, 256, 0, s>>>(dctx, B, emb, D, K, idx, w, ds);
+    SLDM_LAUNCH_CHECK("k_map_attention_bwd_ds_wide");
+    k_map_attention_bwd_mlp_wide<<<mgrid, 256, 0, s>>>(dist, ds, B, K, per_cta, W1, b1, W2, H, HL, part);
+    SLDM_LAUNCH_CHECK("k_map_attention_bwd_mlp_wide");
+  } else {
+#define SLDM_MB(KK) do { if (vec) k_map_attention_bwd_ds<KK, 8><<<ds_grid(k_map_attention_bwd_ds<KK, 8>, 4), 256, 0, s>>>(dctx, B, emb, D, idx, w, ds); \
+                         else k_map_attention_bwd_ds<KK, 32><<<ds_grid(k_map_attention_bwd_ds<KK, 32>, 1), 256, 0, s>>>(dctx, B, emb, D, idx, w, ds); } while (0)
+    switch (K) {
+      case 1: SLDM_MB(1); break; case 2: SLDM_MB(2); break; case 3: SLDM_MB(3); break; case 4: SLDM_MB(4); break;
+      case 5: SLDM_MB(5); break; case 6: SLDM_MB(6); break; case 7: SLDM_MB(7); break; default: SLDM_MB(8); break;
+    }
+#undef SLDM_MB
+    SLDM_LAUNCH_CHECK("k_map_attention_bwd_ds");
+    k_map_attention_bwd_mlp<<<mgrid, 256, 0, s>>>(dist, ds, B, K, per_cta, W1, b1, W2, H, HL, part);
+    SLDM_LAUNCH_CHECK("k_map_attention_bwd_mlp");
+  }
   k_map_attention_reduce<<<ceil_div(3 * H + 1, 8), 256, 0, s>>>(part, mgrid, H, dW1, db1, dW2, db2);
   SLDM_LAUNCH_CHECK("k_map_attention_reduce");
   if (demb != nullptr && S > 0) {
@@ -837,7 +1200,8 @@ extern "C" int sldm_map_attention_backward(const float* dctx, int64_t B, const f
     const int32_t* mem = csr + L.off[SLDM_CSR_COL_SRC];
     const size_t smb = (size_t)kDembWarps * D * sizeof(float);
 #define SLDM_ME(KK) k_map_attention_demb<KK><<<(unsigned)S, 32 * kDembWarps, smb, s>>>(dctx, D, w, rp, mem, demb)
-    switch (K) {
+    if (K > kMaK) launch_demb_wide<kMaK + 1>(K, (unsigned)S, smb, s, dctx, D, w, rp, mem, demb);
+    else switch (K) {
       case 1: SLDM_ME(1); break; case 2: SLDM_ME(2); break; case 3: SLDM_ME(3); break; case 4: SLDM_ME(4); break;
       case 5: SLDM_ME(5); break; case 6: SLDM_ME(6); break; case 7: SLDM_ME(7); break; default: SLDM_ME(8); break;
     }

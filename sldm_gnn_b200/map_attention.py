@@ -4,7 +4,9 @@ Same constructor `(map_centroids, k_neighbors=5)`, same `forward(vehicle_last_po
 tree (`attn_mlp` = Sequential(Linear(1,16), ReLU, Linear(16,1)); `map_centroids` a non-persistent buffer), so the
 reference's state dicts load strictly.  The arithmetic is one fused kernel of libsldm_sage.so (no [B,S] intermediates)
 with a hand-written backward for the embeddings and the MLP; positions and centroids are data and get no gradient.
-Distance ties are broken towards the lower segment index.  CUDA only.
+Distance ties are broken towards the lower segment index.  CUDA only.  k_neighbors may be 1..32
+(sldm_map_attention_max_k()); up to 8 the kernels keep per-thread lists, above 8 one warp works on each position, with
+the same results contract.  A larger k raises NotImplementedError.
 
 The centroids are a constant of the module, so they are binned once into a uniform grid (sldm_map_grid_build) and every
 forward is a ring search over ~40 candidates per position instead of a scan of all S; the grid is rebuilt when the
@@ -64,7 +66,7 @@ class _MapAttentionFn(torch.autograd.Function):
                 wsb = int(lib.sldm_csr_workspace_bytes(nodes, B * K))
                 ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
                 check(lib.sldm_csr_build_pairs(None, idx.data_ptr(), B * K, nodes, csr_buf.data_ptr(), ws.data_ptr(), wsb, _stream(dev)))
-            wsb2 = int(lib.sldm_map_attention_workspace_bytes(B, H))
+            wsb2 = int(lib.sldm_map_attention_workspace_bytes_k(B, H, K))
             ws2 = torch.empty(max(wsb2, 1), dtype=torch.uint8, device=dev)
             check(lib.sldm_map_attention_backward(_ptr(dout), B, _ptr(emb), S, D, K, _ptr(idx), _ptr(dist), _ptr(w),
                                                   _ptr(W1), _ptr(b1), _ptr(W2), H, _ptr(csr_buf), nodes,
