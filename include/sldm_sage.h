@@ -317,7 +317,9 @@ int     sldm_map_attention_backward(const float* dctx, int64_t B, const float* e
  * frames where both are present give an edge iff their minimum is <= m_radius, with attributes
  * [min, max, mean, mean of squares]; edges come out in (i, j) lexicographic order like the reference's lists.
  *   count: counts[V], offsets[V+1]; the caller reads E = offsets[V] (device -> host) to size the outputs,
- *   fill : edge_index int64 [2,E], edge_attr fp32 [E,4].      T <= 128.
+ *   fill : edge_index int64 [2,E], edge_attr fp32 [E,4].
+ * Any T >= 0 (means are numpy's float32 pairwise sums bit for bit, at every length); F >= 5; V < 2^24; E must fit
+ * the int32 offsets.  Neither pass uses shared memory or per-thread storage that grows with T.
  */
 int sldm_edge_build_count(const float* x, int64_t V, int32_t T, int32_t F, float m_radius,
                           int32_t* counts, int32_t* offsets, sldm_stream_t stream);
